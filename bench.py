@@ -41,6 +41,24 @@ METRIC = "train frames/sec (fwd+bwd render)"
 UNIT = "frames/s"
 
 
+DUMP_BYTES = 64 * 1024 * 1024
+
+
+def dump_outputs(path, arrays):
+    """--dump-outputs: write each device tensor of `arrays` ({name: tensor}) to path/<name>.npy as float32.  The files total at most
+    DUMP_BYTES: an array over its equal share keeps a fixed sample of its rows (np.random.default_rng(0), sorted), the same rows in
+    every run of the same workload, so that two builds can be compared file for file."""
+    os.makedirs(path, exist_ok=True)
+    share = DUMP_BYTES // max(1, len(arrays))
+    for name, t in arrays.items():
+        a = t.detach().float().cpu().numpy()
+        a = a.reshape(a.shape[0], -1) if a.ndim > 1 else a.reshape(-1, 1)
+        row_bytes = a.shape[1] * 4
+        if a.nbytes > share:
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], share // row_bytes, replace=False))]
+        np.save(os.path.join(path, name + ".npy"), np.ascontiguousarray(a, np.float32))
+
+
 def load_peaks():
     path = os.path.join(ROOT, "MEASURED_PEAKS.json")
     if os.path.exists(path):
@@ -427,6 +445,7 @@ def run_grt(args, rank, local_rank, world, dev, dist, sub=False):
     d_nrm = torch.zeros((1, H, W, 3), device=dev)
     flush = torch.empty(256 * 1024 * 1024 // 4, dtype=torch.float32, device=dev)
     stage = {"build_bvh": [], "trace": [], "trace_bwd": []}
+    last = {}  # the latest step's outputs (fresh tensors every step)
 
     def view_of(step):
         return (step * world + rank) % n_views
@@ -443,6 +462,7 @@ def run_grt(args, rank, local_rank, world, dev, dist, sub=False):
         if timed:
             evs[2].record()
         dp, ds = ot.trace_bwd(step, c2w, rays_o, rays_d, feat, alpha, hit, nrm, particles, sph, d_rgb, d_alpha, d_dist, d_nrm, 0, sc.sph_degree, 0.001)
+        last.update(rgb=feat, alpha=alpha, dist=hit, normals=nrm, hits=hits, visibility=vis, d_particles=dp, d_sph=ds)
         if timed:
             evs[3].record()
             torch.cuda.synchronize(dev)
@@ -474,6 +494,8 @@ def run_grt(args, rank, local_rank, world, dev, dist, sub=False):
         step_device(n_warm + s)
         ev[s][1].record()
     barrier()
+    if args.dump_outputs and rank == 0 and not sub:
+        dump_outputs(args.dump_outputs, last)
     clocks = sampler.stop() if (rank == 0 and not sub) else None
     total_ms = torch.tensor([float(sum(a.elapsed_time(b) for a, b in ev))], device=dev, dtype=torch.float64)
     if world > 1:
@@ -598,12 +620,12 @@ def run_grt(args, rank, local_rank, world, dev, dist, sub=False):
         dist.destroy_process_group()
 
 
-def gut_device_loop(torch, dist, args, rank, world, dev, workload, steps, warmup, stage_pass=True, zero_dist_grad=False):
+def gut_device_loop(torch, dist, args, rank, world, dev, workload, steps, warmup, stage_pass=True, zero_dist_grad=False, dump_dir=None):
     """Device-timed 3DGUT loop on one workload: `warmup` untimed + `steps` timed view-steps per rank (one view forward + backward each), L2
     flushed between steps, per-step CUDA events, MAX over ranks.  With world > 1 every rank renders a different camera and the gradients are
     summed every `--accumulate` view-steps (a step's batch = accumulate x world views; DESIGN.md section 8): `compact` all-gathers each
     view's [N,4] radiance gradient asynchronously (it overlaps the next view's render), all-reduces the accumulated [N,12] once and rebuilds
-    the [N,48] SH gradient; `allreduce` all-reduces [N,60] once per batch."""
+    the [N,48] SH gradient; `allreduce` all-reduces [N,60] once per batch.  `dump_dir`: rank 0 writes the last timed step's outputs there."""
     import scenes
     import threedgut_tracer
     from threedgut_tracer.tracer import fromOpenCVPinholeCameraModelParameters, ShutterType
@@ -642,11 +664,13 @@ def gut_device_loop(torch, dist, args, rank, world, dev, workload, steps, warmup
         compact = view_parallel.CompactGradientExchange(raster, n, dev, views_per_rank=V)
         pos_table = np.stack([raster.sensor_position(sensor, p, p, W, H) for p in poses]).astype(np.float32)  # every rank knows every pose
     xev = []  # (start, end) events around the exposed part of the exchange, filled only in the stage pass
+    last = {}  # the latest step's forward outputs (fresh tensors every step)
 
     def step_device(step, time_exchange=False):
         pose = poses[view_of(step)]
         slot = step % V
         rgba, dst, hits, vis = raster.trace(step, sc.sph_degree, particles, sph, rays_o, rays_d, None, sensor, 0, 1, pose, pose)
+        last.update(rgba=rgba, dist=dst, hits=hits, visibility=vis)
         if compact is not None:
             # 64 B instead of 240 B per Gaussian on the wire: all-reduce d_particles, all-gather the radiance gradients, rebuild d_sph
             raster.trace_bwd_compact(step, sc.sph_degree, particles, sph, rays_o, rays_d, None, sensor, 0, 1, pose, pose, rgba, d_rgba, dst,
@@ -698,9 +722,13 @@ def gut_device_loop(torch, dist, args, rank, world, dev, workload, steps, warmup
     for s_ in range(steps):
         flush.fill_(float(s_))  # L2 flush between timed iterations, outside the per-step event pair
         ev[s_][0].record()
-        step_device(warmup + s_)
+        grads = step_device(warmup + s_)
         ev[s_][1].record()
     barrier()
+    if dump_dir is not None and rank == 0:  # before the stage pass below reuses the gradient buffers
+        if grads is not None:
+            last.update(d_particles=grads[0], d_sph=grads[1])
+        dump_outputs(dump_dir, last)
     step_ms = np.array([a.elapsed_time(b) for a, b in ev], dtype=np.float64)
     total_ms = torch.tensor([float(step_ms.sum())], device=dev, dtype=torch.float64)
     if world > 1:
@@ -754,6 +782,9 @@ def main():
     ap.add_argument("--profile-host", default=None, help="write a cProfile of the end-to-end loop's host side to this file (diagnostic; the e2e number of such a run is not a bench value)")
     ap.add_argument("--sub-records", default="train_default,c3,c4", help="which sub-records the default c2 line carries (comma list)")
     ap.add_argument("--no-sub-records", action="store_true", help="skip the c3 (6M Gaussians) and c4 (3DGRT) sub-records of the default c2 line")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed (rendered images, visibility, gradients) as "
+                         "DIR/<name>.npy, float32, at most 64 MiB in all (larger arrays keep a fixed sample of rows); inputs are seeded")
     args = ap.parse_args()
 
     rank = int(os.environ.get("RANK", "0"))
@@ -786,7 +817,8 @@ def main():
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()  # runs through warm-up and the timed region (both under load)
-    main_run = gut_device_loop(torch, dist, args, rank, world, dev, args.workload, args.steps, args.warmup, stage_pass=True)
+    main_run = gut_device_loop(torch, dist, args, rank, world, dev, args.workload, args.steps, args.warmup, stage_pass=True,
+                               dump_dir=args.dump_outputs)
     clocks = sampler.stop() if rank == 0 else None
     o = main_run["objs"]
     sc, tracer, raster, ctx, particles, sph, rays_o, rays_d, poses, d_rgba, d_dist, flush, view_of = (

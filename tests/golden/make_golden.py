@@ -1,10 +1,11 @@
 #!/usr/bin/env python
 """Regenerates tests/golden/*.npz from the REFERENCE's own hand-written CUDA math compiled for the host
-(oracle/_ref/libgut_ref.so <- /root/reference sources, see oracle/ref_gut.cpp).  Run in the build container:
+(oracle/_ref/libgut_ref.so, built from the reference's sources by `make -C oracle ref`, see oracle/ref_gut.cpp):
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py [fixture ...]
+    python tests/golden/make_golden.py --gpu     # the reference's own kernels on a GPU (oracle/_ref/libgut_ref_cuda.so, `make -C oracle refcuda`)
 
-The fixtures are what pins oracle/gut_oracle.c on machines where /root/reference does not exist (the GPU box)."""
+The fixtures pin oracle/gut_oracle.c without the reference's sources at hand."""
 import os
 import sys
 
@@ -12,10 +13,11 @@ import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
-for p in (ROOT, os.path.join(ROOT, "3dgrut_b200")):
+for p in (ROOT, os.path.join(ROOT, "3dgrut_b200"), os.path.dirname(HERE)):
     sys.path.insert(0, p)
 
 import scenes  # noqa: E402
+from helpers import array_sha  # noqa: E402
 from oracle import gut_ref as gr  # noqa: E402
 
 
@@ -110,11 +112,144 @@ def sph():
     np.savez_compressed(os.path.join(HERE, "gut_sph_ref.npz"), coeffs=c, dirs=d, rgb=out)
 
 
+def _digests(out, case, arrays):
+    out[f"{case}__sha"] = np.array([f"{k}={array_sha(v)}" for k, v in arrays.items()])
+
+
+def _projection_record(out, case, rf, keys, vals):
+    """What tests/test_oracle_vs_ref.py compares bit for bit, as SHA-256 digests (tile counts and visibility in full)."""
+    out[f"{case}__tiles_count"] = rf["tiles_count"]
+    out[f"{case}__visibility"] = rf["visibility"].astype(np.int8)
+    order = np.argsort(keys, kind="stable")
+    _digests(out, case, dict({k: rf[k] for k in ("depth", "proj_pos", "conic_opacity", "extent")}, rgb_visible=rf["rgb"][rf["tiles_count"] > 0],
+                             keys=keys, vals=vals, sorted_keys=keys[order], sorted_vals=vals[order]))
+
+
+def ref_cases():
+    """The reference's side of every case of tests/test_oracle_vs_ref.py, on the same inputs (gut_ref_cases.npz)."""
+    import test_oracle_vs_ref as t
+
+    out = {}
+    sc = scenes.scene_c1(bands=True)
+    for i in range(6):
+        pose = scenes.pose7_from_c2w(sc.camera(i, 6))
+        rf = gr.project(sc.particles, sc.sph, 3, sc.width, sc.height, [sc.fx, sc.fy], [sc.cx, sc.cy], pose, pose)
+        keys, vals = gr.expand(sc.width, sc.height, rf["tiles_count"], rf["proj_pos"], rf["conic_opacity"], rf["extent"], rf["depth"])
+        _projection_record(out, f"pinhole{i}", rf, keys, vals)
+    f = 1.2 * sc.width
+    gr.set_camera_model(t.FISHEYE)
+    try:
+        for i in range(4):
+            pose = scenes.pose7_from_c2w(sc.camera(i, 4))
+            rf = gr.project(sc.particles, sc.sph, 3, sc.width, sc.height, [f, f], [sc.cx, sc.cy], pose, pose)
+            keys, vals = gr.expand(sc.width, sc.height, rf["tiles_count"], rf["proj_pos"], rf["conic_opacity"], rf["extent"], rf["depth"])
+            _projection_record(out, f"fisheye{i}", rf, keys, vals)
+    finally:
+        gr.set_camera_model(None)
+    for poly in (0, 1):
+        ft = t._ftheta(sc.width, sc.height, poly)
+        gr.set_ftheta(ft)
+        try:
+            for i in range(3):
+                pose = scenes.pose7_from_c2w(sc.camera(i, 3))
+                rf = gr.project(sc.particles, sc.sph, 3, sc.width, sc.height, [1.0, 1.0], list(ft["principal"]), pose, pose)
+                keys, vals = gr.expand(sc.width, sc.height, rf["tiles_count"], rf["proj_pos"], rf["conic_opacity"], rf["extent"], rf["depth"])
+                _projection_record(out, f"ftheta{poly}_{i}", rf, keys, vals)
+        finally:
+            gr.set_camera_model(None)
+    p0 = scenes.pose7_from_c2w(sc.camera(1, 40))
+    p1 = scenes.pose7_from_c2w(sc.camera(2, 40))
+    for model in ("pinhole", "fisheye"):
+        fe = t.FISHEYE if model == "fisheye" else None
+        f = 1.2 * sc.width if model == "fisheye" else sc.fx
+        for kind in (1, 2, 3, 4):
+            gr.set_camera_model(fe)
+            gr.set_rolling_shutter(kind)
+            try:
+                rf = gr.project(sc.particles, sc.sph, 3, sc.width, sc.height, [f, f], [sc.cx, sc.cy], p0, p1)
+            finally:
+                gr.set_rolling_shutter(0)
+                gr.set_camera_model(None)
+            case = f"shutter_{model}{kind}"
+            out[f"{case}__tiles_count"] = rf["tiles_count"]
+            _digests(out, case, {k: rf[k] for k in ("depth", "proj_pos", "conic_opacity", "extent")})
+    sc8 = scenes.scene_c1()
+    for i in range(8):
+        pose = scenes.pose7_from_c2w(sc8.camera(i, 8))
+        for k, v in zip(("view", "inv", "pos"), gr.sensor_matrices(pose, pose)):
+            out[f"sensor{i}__{k}"] = v
+    for degree in (2, 4):
+        # the same random stream as the test; only accepted hits carry values (a rejected one is compared by its flag)
+        rng = np.random.default_rng(degree)
+        acc_all, rows = [], []
+        for _ in range(1500):
+            p, ro, rd = t._random_hit_case(rng)
+            rgb = rng.uniform(0, 1, 3).astype(np.float32)
+            T, C0, D = float(rng.uniform(0.05, 1)), rng.uniform(0, 0.5, 3).astype(np.float32), float(rng.uniform(0, 2))
+            acc, T1, _, D1 = gr.hit_fwd(degree, ro, rd, p, rgb, T, C0, D)
+            Tint, Cint, Dint = T * rng.uniform(0.001, 0.9), C0 + rng.uniform(0.1, 1, 3).astype(np.float32), D + rng.uniform(0.1, 3)
+            Tg, Cg, Dg = float(rng.normal()), rng.normal(size=3).astype(np.float32), float(rng.normal())
+            g, rg, Tb, _, _ = gr.hit_bwd(degree, ro, rd, p, rgb, 1e-4, Tint, T, Tg, Cint, C0, Cg, Dint, D, Dg)
+            acc_all.append(acc)
+            if acc:
+                rows.append(np.concatenate([[T1, D1], g[:11], rg, [Tb]]))
+        out[f"hits{degree}__accepted"] = np.asarray(acc_all, np.int8)
+        out[f"hits{degree}__rows"] = np.asarray(rows, np.float32)  # T after, D after, d particle[:11], d rgb, T adjoint
+    rng = np.random.default_rng(5)
+    sph_out = []
+    for deg in range(4):
+        for _ in range(50):
+            c = rng.normal(size=48).astype(np.float32)
+            d = rng.normal(size=3)
+            d = (d / np.linalg.norm(d)).astype(np.float32)
+            sph_out.append(gr.sph(deg, c, d, clamped=False))
+    out["sph__rgb"] = np.stack(sph_out)
+    np.savez_compressed(os.path.join(HERE, "gut_ref_cases.npz"), **out)
+
+
+def _run_reference_gpu(sc, pose, d_rgba, d_dist):
+    """One forward + backward frame through the reference's own 3DGUT kernels (oracle/_ref/libgut_ref_cuda.so) on cuda:0."""
+    import torch
+
+    from oracle import gut_ref_cuda as grc
+
+    dev = torch.device("cuda", 0)
+    t = lambda a: torch.from_numpy(np.ascontiguousarray(a)).to(dev)  # noqa: E731
+    ro, rd = sc.rays()
+    particles, sph, tro, trd = t(sc.particles), t(sc.sph), t(ro), t(rd)
+    rr = grc.ReferenceRaster()
+    s = torch.cuda.current_stream(dev).cuda_stream
+    rgba, dist, hits, vis = rr.trace(torch, s, 0, sc.sph_degree, particles, sph, sc.width, sc.height, sc.fx, sc.fy, sc.cx, sc.cy, pose, tro, trd)
+    torch.cuda.synchronize()
+    tiles = ((sc.width + 15) // 16) * ((sc.height + 15) // 16)
+    dbg = {k: rr.debug(k, sc.n, tiles) for k in ("tiles_count", "sorted_keys", "sorted_values", "ranges", "depth")}
+    dp, ds = rr.trace_bwd(torch, s, 0, sc.sph_degree, particles, sph, sc.width, sc.height, sc.fx, sc.fy, sc.cx, sc.cy, pose, tro, trd, rgba,
+                          t(d_rgba), dist, t(d_dist))
+    torch.cuda.synchronize()
+    out = dict(rgba=rgba.cpu().numpy(), dist=dist.cpu().numpy(), hits=hits.cpu().numpy(), dp=dp.cpu().numpy(), ds=ds.cpu().numpy(), **dbg)
+    rr.close()
+    return out
+
+
+def ref_gpu():
+    """The reference's GPU frames of tests/test_ref_cuda_gpu.py, reduced by helpers.frame_record (ref_gpu_<case>.npz).  Needs a GPU."""
+    import test_ref_cuda_gpu as t
+    from helpers import frame_record
+
+    for case, (make_scene, cam_index, n_cams) in t.CASES.items():
+        sc = make_scene()
+        _, pose, d_rgba, d_dist = t.frame_inputs(sc, cam_index, n_cams)
+        np.savez_compressed(os.path.join(HERE, f"ref_gpu_{case}.npz"), **frame_record(_run_reference_gpu(sc, pose, d_rgba, d_dist)))
+
+
+CPU_FIXTURES = dict(projection=projection, projection_fisheye=projection_fisheye, projection_ftheta=projection_ftheta, hits=hits, sph=sph,
+                    ref_cases=ref_cases)
+
 if __name__ == "__main__":
-    assert gr.available(), "oracle/_ref could not be built (needs /root/reference)"
-    projection()
-    projection_fisheye()
-    projection_ftheta()
-    hits()
-    sph()
+    if sys.argv[1:] == ["--gpu"]:
+        ref_gpu()
+    else:
+        assert gr.available(), "oracle/_ref could not be built (needs the reference sources, see oracle/Makefile)"
+        for name in sys.argv[1:] or list(CPU_FIXTURES):
+            CPU_FIXTURES[name]()
     print("golden fixtures written to", HERE)

@@ -1,4 +1,7 @@
 """Shared helpers of the parity tests."""
+import hashlib
+import zlib
+
 import numpy as np
 
 import scenes
@@ -49,6 +52,40 @@ def image_error_report(name, got, ref, atol=1e-4):
 def rel_l2(a, b):
     a, b = np.asarray(a, np.float64), np.asarray(b, np.float64)
     return float(np.linalg.norm(a - b) / max(np.linalg.norm(b), 1e-30))
+
+
+def array_sha(a):
+    """SHA-256 of an array's bytes: golden fixtures store this instead of large arrays that must match bit for bit."""
+    return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
+
+
+def spread_sample(n, k):
+    """min(n, k) distinct indices of range(n), spread over it by a fixed permutation (multiplication by a prime > n), sorted."""
+    return np.sort((np.arange(min(n, k), dtype=np.int64) * 2654435761) % n)
+
+
+def frame_record(f, grad_rows=None):
+    """A forward + backward frame reduced to what fits a golden fixture (tests/test_ref_cuda_gpu.py): tile counts, depth, pixels and
+    gradient rows on fixed samples; per-tile CRC32 of the sorted value lists; SHA-256 digests of the full integer streams.  `grad_rows`
+    defaults to a sample of the particles with a non-zero position / density / rotation / scale gradient."""
+    n = f["tiles_count"].shape[0]
+    rgba = np.asarray(f["rgba"], np.float32).reshape(-1, 4)
+    dist = np.asarray(f["dist"], np.float32).reshape(-1)
+    hits = np.asarray(f["hits"], np.float32).reshape(-1)
+    dp, ds = np.asarray(f["dp"], np.float32), np.asarray(f["ds"], np.float32)
+    if grad_rows is None:
+        live = np.flatnonzero(np.any(dp[:, :11] != 0, axis=1))
+        grad_rows = live[spread_sample(live.size, 128)]
+    ranges, values = np.asarray(f["ranges"], np.int64).reshape(-1, 2), np.asarray(f["sorted_values"], np.uint32)
+    pi, di, px, hx = spread_sample(n, 8192), spread_sample(n, 1024), spread_sample(dist.size, 2048), spread_sample(dist.size, 8192)
+    return dict(tiles_count=np.asarray(f["tiles_count"], np.uint32)[pi], depth=np.asarray(f["depth"], np.float32)[di],
+                tile_crc=np.array([zlib.crc32(values[a:b].tobytes()) for a, b in ranges], np.uint32),
+                rgba=rgba[px], dist=dist[px], hits=hits[hx], grad_rows=grad_rows, dp=dp[grad_rows], ds=ds[grad_rows],
+                tiles_total=np.int64(np.asarray(f["tiles_count"], np.int64).sum()),
+                dist_scale=np.float64(max(1.0, float(np.abs(dist[dist < 1e5]).max()))),
+                sha=np.array([f"{k}={array_sha(np.asarray(f[k], t))}" for k, t in (("tiles_count", np.uint32), ("depth", np.float32),
+                                                                                    ("sorted_keys", np.uint64), ("sorted_values", np.uint32),
+                                                                                    ("ranges", np.uint32))]))
 
 
 def frac_within(a, b, atol):

@@ -44,7 +44,7 @@ EXPORTS = [
     "gutb200_debug_copy", "gutb200_collect_times", "gutb200_collect_stage_times", "gutb200_set_timings", "gutb200_launch_count",
     "gutb200_backward_compact", "gutb200_sph_grad_from_views", "gutb200_camera_position",
     "gutb200_debug_work_counters", "gutb200_debug_fma_peak",
-    "gutb200_selective_adam_update", "gutb200_gaussian_adam_step",  # bound in optimizers/__init__.py
+    "gutb200_selective_adam_update", "gutb200_gaussian_adam_step", "gutb200_gaussian_adam_step_reg",  # bound in optimizers/__init__.py
     "gutb200_image_loss_scratch_bytes", "gutb200_image_loss",  # bound in losses.py
 ]
 

@@ -23,9 +23,11 @@ def _lib():
         vp, i64, i32, f32 = C.c_void_p, C.c_int64, C.c_int32, C.c_float
         lib.gutb200_selective_adam_update.argtypes = [vp, vp, vp, vp, vp, vp, f32, f32, f32, f32, i64, i64]
         lib.gutb200_selective_adam_update.restype = C.c_int
-        lib.gutb200_gaussian_adam_step.argtypes = [vp, i64, C.POINTER(vp), C.POINTER(vp), C.POINTER(vp), C.POINTER(f32), f32, f32, f32, i64, i32,
-                                                   vp, vp, vp]
+        step_args = [vp, i64, C.POINTER(vp), C.POINTER(vp), C.POINTER(vp), C.POINTER(f32), f32, f32, f32, i64, i32, vp, vp, vp]
+        lib.gutb200_gaussian_adam_step.argtypes = step_args
         lib.gutb200_gaussian_adam_step.restype = C.c_int
+        lib.gutb200_gaussian_adam_step_reg.argtypes = step_args + [f32, f32, vp]
+        lib.gutb200_gaussian_adam_step_reg.restype = C.c_int
         lib._optim_bound = True
     return lib
 
@@ -83,7 +85,10 @@ class FusedGaussianAdam:
 
     params: dict name -> raw (pre-activation) leaf tensor for the six GROUPS; lrs: dict name -> learning rate (mutable: schedulers
     write `opt.lrs["positions"] = ...`).  step(d_particles, d_sph, visibility=None) consumes the renderer's gradients
-    (Tracer / SplatRaster.trace_bwd outputs, or the view-parallel exchange's) -- no autograd pass over the activations is needed."""
+    (Tracer / SplatRaster.trace_bwd outputs, or the view-parallel exchange's) -- no autograd pass over the activations is needed.
+    step(..., lambda_opacity, lambda_scale) also applies the reference's opacity / scale regularisers (trainer.py:722-739) in the same
+    launch; reg_loss, a float32 CUDA tensor of two elements, then receives their unweighted values (mean sigmoid(density), mean
+    exp(scale)) before the update."""
 
     def __init__(self, params: dict, lrs: dict, betas=(0.9, 0.999), eps=1e-15, selective=False):
         # the dict itself is kept (not copied) when it holds exactly the six groups: densification replaces the tensors inside it
@@ -115,7 +120,8 @@ class FusedGaussianAdam:
         return arr
 
     @torch.no_grad()
-    def step(self, d_particles: torch.Tensor, d_sph: torch.Tensor, visibility: torch.Tensor | None = None):
+    def step(self, d_particles: torch.Tensor, d_sph: torch.Tensor, visibility: torch.Tensor | None = None, lambda_opacity: float = 0.0,
+             lambda_scale: float = 0.0, reg_loss: torch.Tensor | None = None):
         _check(d_particles, "d_particles")
         _check(d_sph, "d_sph")
         self._validate()  # the tensors may have been replaced (densification); moments must have followed
@@ -134,13 +140,22 @@ class FusedGaussianAdam:
             vis = vis.contiguous()
             _check(vis, "visibility")
             vis_ptr = vis.data_ptr()
+        lambda_opacity, lambda_scale = float(lambda_opacity), float(lambda_scale)
+        regularised = lambda_opacity != 0.0 or lambda_scale != 0.0 or reg_loss is not None
+        if reg_loss is not None:
+            _check(reg_loss, "reg_loss")
+            if reg_loss.numel() < 2 or reg_loss.device != d_particles.device:
+                raise RuntimeError("reg_loss must hold two floats on the gradients' device")
         self.steps += 1
         dev = d_particles.device
         lr = (C.c_float * 6)(*[self.lrs[k] for k in GROUPS])
         stream = torch.cuda.current_stream(dev).cuda_stream
+        args = (stream, self.n, self._array({k: t.data for k, t in self.params.items()}), self._array(self.exp_avg), self._array(self.exp_avg_sq),
+                lr, self.betas[0], self.betas[1], self.eps, self.steps, int(self.selective), d_particles.data_ptr(), d_sph.data_ptr(), vis_ptr)
         with torch.cuda.device(dev):
-            rc = _lib().gutb200_gaussian_adam_step(stream, self.n, self._array({k: t.data for k, t in self.params.items()}),
-                                                   self._array(self.exp_avg), self._array(self.exp_avg_sq), lr, self.betas[0], self.betas[1],
-                                                   self.eps, self.steps, int(self.selective), d_particles.data_ptr(), d_sph.data_ptr(), vis_ptr)
+            if regularised:
+                rc = _lib().gutb200_gaussian_adam_step_reg(*args, lambda_opacity, lambda_scale, None if reg_loss is None else reg_loss.data_ptr())
+            else:
+                rc = _lib().gutb200_gaussian_adam_step(*args)
         if rc != 0:
-            raise RuntimeError(f"gutb200_gaussian_adam_step failed ({rc})")
+            raise RuntimeError(f"gutb200_gaussian_adam_step{'_reg' if regularised else ''} failed ({rc})")

@@ -122,6 +122,16 @@ int gutb200_selective_adam_update(void* stream, float* param, const float* grad,
 int gutb200_gaussian_adam_step(void* stream, int64_t n, float* const* params6, float* const* exp_avg6, float* const* exp_avg_sq6,
                                const float* lr6, float b1, float b2, float eps, int64_t step, int32_t selective, const float* d_particles,
                                const float* d_sph, const float* visibility);
+/* gutb200_gaussian_adam_step plus the opacity and scale regularisers of the reference's loss (threedgrut/trainer.py:722-739):
+ *   loss += lambda_opacity * mean|sigmoid(density)|  +  lambda_scale * mean|exp(scale)|      (means over [n,1] and [n,3])
+ * Their gradients are added to the density / scale gradients inside the launch, once per call: called after the view-parallel
+ * exchange, every replica adds the same term.  Selective mode masks rows exactly as gutb200_gaussian_adam_step does (invisible rows get
+ * no update, as the reference's SelectiveAdam drops their regulariser gradient too).  reg_loss2: NULL, or a device float[2] that is
+ * zeroed on `stream` and receives (mean sigmoid(density), mean exp(scale)) of the parameters BEFORE the update; the summation order,
+ * and so the last bits of these two values, may vary between runs, the parameters never do. */
+int gutb200_gaussian_adam_step_reg(void* stream, int64_t n, float* const* params6, float* const* exp_avg6, float* const* exp_avg_sq6,
+                                   const float* lr6, float b1, float b2, float eps, int64_t step, int32_t selective, const float* d_particles,
+                                   const float* d_sph, const float* visibility, float lambda_opacity, float lambda_scale, float* reg_loss2);
 
 /* Image loss of the training step and its gradient (SURVEY.md 8f row 3): loss = lambda_l1 mean|x - y| + lambda_ssim (1 - SSIM(x, y))
  * (threedgrut/trainer.py:698-739, model/losses.py:20-33 -> fused_ssim(..., padding="valid"), third-party fused-ssim @ 1272e21).
